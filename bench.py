@@ -27,6 +27,7 @@ if ROOT not in sys.path:
 ALGO_BYTES_PER_TEXEL = 40.0       # SURVEY 8d: read h0 16 + read foam texel 8 + write 2 x RGBA16F 16
 METRIC = "ifft_cascades_per_sec"
 UNIT = "cascades/s"
+DUMP_BYTES = 32 * 2**20           # --dump-outputs budget: one 1024x1024 cascade (both maps as float32) fits it
 
 DEMO_SETS = [   # main.tscn:43-83 + wave_cascade_parameters.gd defaults (SURVEY appendix B)
     dict(tile_length=(88.0, 88.0), displacement_scale=1.0, normal_scale=1.0, wind_speed=10.0, wind_direction=20.0,
@@ -208,6 +209,20 @@ def workload_config(args, world: int) -> dict:
                 (ALGO_BYTES_PER_TEXEL + 64) * C * N * N / 2**20)}
 
 
+def sample_outputs(gen, C: int, N: int) -> dict:
+    """What the last update_all() handed its caller: both RGBA16F maps, widened to float32 (exact), of every resident
+    cascade when they fit DUMP_BYTES, else of a fixed seeded choice of cascades (in ascending order)."""
+    import numpy as np
+    k = max(1, min(C, DUMP_BYTES // (2 * N * N * 4 * 4)))
+    pick = np.sort(np.random.default_rng(0).choice(C, size=k, replace=False))
+    out = {"displacement_map": np.empty((k, N, N, 4), np.float32), "normal_map": np.empty((k, N, N, 4), np.float32)}
+    for j, c in enumerate(pick):
+        d, n = gen.maps_to_host(int(c), 1)
+        out["displacement_map"][j] = d[0]
+        out["normal_map"][j] = n[0]
+    return out
+
+
 def run_reference(args, rank: int):
     if rank != 0:
         return
@@ -294,6 +309,9 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=20.0, help="CPU-baseline sample budget inside the native arm")
     ap.add_argument("--reference-seconds", type=float, default=240.0, help="time budget of the whole --impl reference run")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the maps of the last timed step (rank 0's cascades, a seeded sample of them beyond 32 MiB) "
+                         "as DIR/<name>.npy in float32")
     ap.add_argument("--workload", default="cfg2", choices=["cfg2", "cfg4-strong"],
                     help="cfg2: BASELINE configs[1], weak scaling (default, the driver's contract); cfg4-strong: BASELINE configs[3], "
                          "1024x1024 x 8 cascades split over the GPUs (8/4/2/1 per GPU), strong scaling")
@@ -383,6 +401,8 @@ def main():
     for _ in range(args.steps):
         gen.update_all(delta, params)
     ms = gen.timer_stop()
+    # read before the untimed updates below advance the state
+    outputs = sample_outputs(gen, C, N) if args.dump_outputs and rank == 0 else None
     if len(sampler.samples) < 5:
         # the timed region is only tens of milliseconds and the submitting thread rarely yields the GIL: keep the
         # same workload running (untimed) for ~0.5 s so that NVML sees the clocks under this load
@@ -452,6 +472,11 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     peak_gbs, peak_src = measured_peaks()
     traffic, traffic_src = ncu_traffic()

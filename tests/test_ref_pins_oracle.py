@@ -2,49 +2,119 @@
 
 oracle/_ref/libocean_ref.so is the reference's OWN six compute shaders (assets/shaders/compute/*.glsl, text unmodified
 apart from the lexical plumbing listed in oracle/ref/glsl2cpp.py) compiled for the CPU and driven like
-assets/water/wave_generator.gd drives them (oracle/pyref.py).  These tests assert that oracle/ocean_oracle.c -- the C
-restatement every GPU parity test compares the CUDA path against -- reproduces the shaders' outputs BIT FOR BIT: the
-butterfly table, the spectrum texture, both halves of the FFT buffer and both RGBA16F maps, for the BASELINE configs that
-a CPU finishes in seconds, the parameter corners, the update/_process interleaving and every numeric-policy mode.
+assets/water/wave_generator.gd drives them (oracle/pyref.py).  tools/make_golden.py ran every scenario below through those
+shaders and stored a SHA-256 of each resource at every checkpoint in tests/golden/ref_pins/states.json.  These tests run
+the same scenarios through oracle/ocean_oracle.c -- the C restatement every GPU parity test compares the CUDA path
+against -- and assert that it reproduces the shaders' outputs BIT FOR BIT: the butterfly table, the spectrum texture,
+both halves of the FFT buffer and both RGBA16F maps, for the BASELINE configs that a CPU finishes in seconds, the
+parameter corners, the update/_process interleaving, random parameter draws and every numeric-policy mode.
 """
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
-from conftest import EDGE_CASES, demo_params
+from conftest import EDGE_CASES, ROOT, demo_params
 from oracle import pyoracle as po
 from oracle import pyref as pr
 
-pytestmark = pytest.mark.skipif(not pr.available(), reason="oracle/_ref is neither built nor buildable (no /root/reference)")
+PINS_PATH = os.path.join(ROOT, "tests", "golden", "ref_pins", "states.json")
+RESOURCES = ("butterfly", "spectrum", "fft_buffer", "displacement_map", "normal_map")
 
 MODES = [("detmath_fma", po.MATH_DET, po.CONTRACT_FMA), ("detmath_strict", po.MATH_DET, po.CONTRACT_STRICT),
          ("libm_strict", po.MATH_LIBM, po.CONTRACT_STRICT), ("libm_fma", po.MATH_LIBM, po.CONTRACT_FMA)]
+BASELINE_CONFIGS = [(128, 1, 1), (256, 4, 2)]
+BASELINE_IDS = ["cfg1_128x1", "cfg2_256x4"]
+
+# the two pipelines a scenario can run on: the C oracle, and the reference's shaders (what the pins were recorded from)
+ORACLE = (po.OracleWaveGenerator, po.set_modes)
+REFERENCE = (pr.RefWaveGenerator, pr.set_modes)
+
+
+def state(g) -> dict:
+    """SHA-256 of the bytes of every resource the shaders write."""
+    return {r: hashlib.sha256(np.ascontiguousarray(getattr(g, r)).tobytes()).hexdigest() for r in RESOURCES}
+
+
+def baseline_config(impl, N, C, frames, mode):
+    """BASELINE.json configs[0] and configs[1]: the state after each update."""
+    Gen, set_modes = impl
+    set_modes(mode[1], mode[2])
+    g, p = Gen(N), [demo_params(po.CascadeParams, c) for c in range(C)]
+    states = []
+    for _ in range(frames):
+        g.update_all(1.0 / 50.0, p)
+        states.append(state(g))
+    return {"states": states, "times": [q.time for q in p]}
+
+
+def parameter_corner(impl, name, contract):
+    Gen, set_modes = impl
+    set_modes(po.MATH_DET, contract)
+    g, p = Gen(128), [demo_params(po.CascadeParams, c, **EDGE_CASES[name]) for c in range(2)]
+    for delta in (0.02, 0.0, 0.031):
+        g.update_all(delta, p)
+    return {"states": [state(g)]}
+
+
+def foam_loop(impl):
+    """update()/_process() interleaving (wave_generator.gd:56-63,90-109) and the foam state carried through RGBA16F
+    (fft_unpack.glsl:59-67) over 10 frames of the three demo cascades.  Returns the pin and the generator."""
+    Gen, set_modes = impl
+    set_modes(po.MATH_DET, po.CONTRACT_FMA)
+    N, C = 128, 3
+    g, p = Gen(N), [demo_params(po.CascadeParams, c) for c in range(C)]
+    rng = np.random.default_rng(11)
+    for f in range(10):
+        g.update(1.0 / 50.0 + float(rng.uniform(0, 0.004)), p)
+        for _ in range(int(rng.integers(0, C + 1))):
+            g.process()
+        if f == 4:                                   # a parameter change mid-run regenerates one spectrum
+            p[1].wind_speed = 12.5
+            p[1].should_generate_spectrum = True
+    g.update(0.02, p)
+    while g.pass_num_cascades_remaining:
+        g.process()
+    return {"states": [state(g)]}, g
+
+
+def random_parameters(impl, kw, contract, delta):
+    """One random draw over the @export_range space of wave_cascade_parameters.gd (and beyond): two updates at 128x128."""
+    Gen, set_modes = impl
+    set_modes(po.MATH_DET, contract)
+    g, p = Gen(128), [po.CascadeParams(**kw)]
+    for _ in range(2):
+        g.update_all(delta, p)
+    return {"states": [state(g)]}
+
+
+def random_draw_kwargs(draw: dict) -> dict:
+    """CascadeParams keyword arguments of a stored random draw (JSON keeps the tuples as lists)."""
+    return {k: tuple(v) if isinstance(v, list) else v for k, v in draw["params"].items()}
+
+
+@pytest.fixture(scope="module")
+def pins():
+    with open(PINS_PATH) as f:
+        return json.load(f)
 
 
 @pytest.fixture(autouse=True)
 def _restore_modes():
     yield
     po.set_modes(po.MATH_DET, po.CONTRACT_FMA)
-    pr.set_modes(po.MATH_DET, po.CONTRACT_FMA)
 
 
-def _bits(a):
-    a = np.ascontiguousarray(a)
-    return a.view(np.uint8)
+def _assert_same_states(got, want, what):
+    assert len(got["states"]) == len(want["states"]), what
+    for i, (g, w) in enumerate(zip(got["states"], want["states"])):
+        for r in RESOURCES:
+            assert g[r] == w[r], f"{what} checkpoint {i}: {r} differs from the reference shaders'"
 
 
-def _assert_same_state(o, r, what):
-    assert np.array_equal(_bits(o.butterfly), _bits(r.butterfly)), f"{what}: butterfly table"
-    assert np.array_equal(_bits(o.spectrum), _bits(r.spectrum)), f"{what}: spectrum texture"
-    assert np.array_equal(_bits(o.fft_buffer), _bits(r.fft_buffer)), f"{what}: fft_buffer (both halves)"
-    assert np.array_equal(o.displacement_map, r.displacement_map), f"{what}: displacement map"
-    assert np.array_equal(o.normal_map, r.normal_map), f"{what}: normal/foam map"
-
-
-def _pair(N, C, **over):
-    return (po.OracleWaveGenerator(N), pr.RefWaveGenerator(N),
-            [demo_params(po.CascadeParams, c, **over) for c in range(C)], [demo_params(po.CascadeParams, c, **over) for c in range(C)])
-
-
+@pytest.mark.skipif(not pr.available(), reason="needs the reference's shaders compiled for the CPU (oracle/_ref)")
 def test_reference_shaders_compiled():
     L = pr.lib()
     for s in pr.SHADERS:
@@ -56,56 +126,25 @@ def test_reference_shaders_compiled():
 
 
 @pytest.mark.parametrize("mode", MODES, ids=[m[0] for m in MODES])
-@pytest.mark.parametrize("N,C,frames", [(128, 1, 1), (256, 4, 2)], ids=["cfg1_128x1", "cfg2_256x4"])
-def test_oracle_reproduces_reference_shaders(N, C, frames, mode):
+@pytest.mark.parametrize("N,C,frames", BASELINE_CONFIGS, ids=BASELINE_IDS)
+def test_oracle_reproduces_reference_shaders(N, C, frames, mode, pins):
     """BASELINE.json configs[0] and configs[1]: every resource bit-identical after each update."""
-    _, math_mode, contract = mode
-    po.set_modes(math_mode, contract)
-    pr.set_modes(math_mode, contract)
-    o, r, po_p, pr_p = _pair(N, C)
-    for f in range(frames):
-        o.update_all(1.0 / 50.0, po_p)
-        r.update_all(1.0 / 50.0, pr_p)
-        _assert_same_state(o, r, f"{mode[0]} frame {f}")
-    assert [p.time for p in po_p] == [p.time for p in pr_p]
+    key = f"baseline/{N}x{C}x{frames}/{mode[0]}"
+    got, want = baseline_config(ORACLE, N, C, frames, mode), pins[key]
+    _assert_same_states(got, want, key)
+    assert got["times"] == want["times"]
 
 
 @pytest.mark.parametrize("name", sorted(EDGE_CASES))
-def test_oracle_reproduces_reference_shaders_on_parameter_corners(name):
-    N = 128
+def test_oracle_reproduces_reference_shaders_on_parameter_corners(name, pins):
     for contract in (po.CONTRACT_FMA, po.CONTRACT_STRICT):
-        po.set_modes(po.MATH_DET, contract)
-        pr.set_modes(po.MATH_DET, contract)
-        o, r, po_p, pr_p = _pair(N, 2, **EDGE_CASES[name])
-        for delta in (0.02, 0.0, 0.031):
-            o.update_all(delta, po_p)
-            r.update_all(delta, pr_p)
-        _assert_same_state(o, r, f"{name} contract={contract}")
+        key = f"corner/{name}/contract{contract}"
+        _assert_same_states(parameter_corner(ORACLE, name, contract), pins[key], key)
 
 
-def test_foam_recurrence_and_scheduling_against_reference_shaders():
-    """update()/_process() interleaving (wave_generator.gd:56-63,90-109) and the foam state carried through RGBA16F
-    (fft_unpack.glsl:59-67) over 10 frames of the three demo cascades."""
-    N, C = 128, 3
-    o, r, po_p, pr_p = _pair(N, C)
-    rng = np.random.default_rng(11)
-    for f in range(10):
-        delta = 1.0 / 50.0 + float(rng.uniform(0, 0.004))
-        o.update(delta, po_p)
-        r.update(delta, pr_p)
-        for _ in range(int(rng.integers(0, C + 1))):
-            o.process()
-            r.process()
-        if f == 4:                                   # a parameter change mid-run regenerates one spectrum
-            for p in (po_p[1], pr_p[1]):
-                p.wind_speed = 12.5
-                p.should_generate_spectrum = True
-    o.update(0.02, po_p)
-    r.update(0.02, pr_p)
-    while o.pass_num_cascades_remaining:
-        o.process()
-        r.process()
-    _assert_same_state(o, r, "foam loop")
+def test_foam_recurrence_and_scheduling_against_reference_shaders(pins):
+    got, o = foam_loop(ORACLE)
+    _assert_same_states(got, pins["foam_loop"], "foam loop")
     assert o.normal_half()[0][..., 3].max() > 0
 
 
@@ -121,32 +160,13 @@ def test_half_conversion_of_the_oracle_equals_the_compilers():
     assert np.array_equal(got, ref)
 
 
-def test_oracle_reproduces_reference_shaders_on_random_parameters():
-    """hypothesis: random draws over the whole @export_range space of wave_cascade_parameters.gd (and beyond), two updates
-    each at 128x128 -- every resource bit-identical between the C oracle and the compiled reference shaders."""
-    from hypothesis import given, settings, HealthCheck
-    from hypothesis import strategies as st
-
-    pos = dict(allow_nan=False, allow_infinity=False)
-    params = st.fixed_dictionaries(dict(
-        tile_length=st.tuples(st.floats(0.5, 4000.0, width=32, **pos), st.floats(0.5, 4000.0, width=32, **pos)),
-        wind_speed=st.floats(0.0001, 60.0, **pos), wind_direction=st.floats(-360.0, 720.0, **pos),
-        fetch_length=st.floats(0.0001, 2000.0, **pos), swell=st.floats(0.0, 2.0, **pos), spread=st.floats(0.0, 1.0, **pos),
-        detail=st.floats(0.0, 1.0, **pos), whitecap=st.floats(0.0, 2.0, **pos), foam_amount=st.floats(0.0, 10.0, **pos),
-        spectrum_seed=st.tuples(st.integers(-2**31, 2**31 - 1), st.integers(-2**31, 2**31 - 1)),
-        time=st.floats(0.0, 50000.0, **pos)))
-
-    @settings(max_examples=12, deadline=None, derandomize=True, suppress_health_check=[HealthCheck.too_slow])
-    @given(kw=params, contract=st.sampled_from([po.CONTRACT_FMA, po.CONTRACT_STRICT]), delta=st.floats(0.0, 0.1, **pos))
-    def run(kw, contract, delta):
-        po.set_modes(po.MATH_DET, contract)
-        pr.set_modes(po.MATH_DET, contract)
-        o, r = po.OracleWaveGenerator(128), pr.RefWaveGenerator(128)
-        a, b = [po.CascadeParams(**kw)], [po.CascadeParams(**kw)]
-        for _ in range(2):
-            o.update_all(delta, a)
-            r.update_all(delta, b)
+def test_oracle_reproduces_reference_shaders_on_random_parameters(pins):
+    """Random draws over the whole @export_range space of wave_cascade_parameters.gd (and beyond), two updates each at
+    128x128 -- every resource bit-identical between the C oracle and the compiled reference shaders.  The draws are
+    hypothesis's (derandomized, 12 examples, boundary values included), stored with the pins by tools/make_golden.py."""
+    draws = pins["random"]
+    assert len(draws) >= 12
+    for d in draws:
+        kw = random_draw_kwargs(d)
         # NaN payloads aside (log(0) at u1 == 0 is reachable in principle), the bytes must agree
-        _assert_same_state(o, r, f"{kw} contract={contract}")
-
-    run()
+        _assert_same_states(random_parameters(ORACLE, kw, d["contract"], d["delta"]), d, f"{kw} contract={d['contract']}")

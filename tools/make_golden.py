@@ -12,6 +12,10 @@ Stored per case: CRC-32 of the full arrays (little-endian bytes) and a strided s
 The map-query vectors (SURVEY 8f row f2) are oracle/sampling.py's (the numpy specification of the water shader's
 sampling contract) evaluated on the reference-produced maps.
 
+It also writes tests/golden/ref_pins/states.json: the scenarios of tests/test_ref_pins_oracle.py run through the same
+shaders in every numeric-policy mode, stored as a SHA-256 of each resource at every checkpoint, which the C oracle must
+reproduce bit for bit.
+
   python tools/make_golden.py            # rewrites tests/golden/
 """
 import json
@@ -77,6 +81,49 @@ def run_case(case):
     return out
 
 
+def random_draws():
+    """The draws hypothesis makes, derandomized (12 examples, boundary values included), over the whole @export_range
+    space of wave_cascade_parameters.gd and beyond."""
+    from hypothesis import HealthCheck, given, settings
+    from hypothesis import strategies as st
+
+    pos = dict(allow_nan=False, allow_infinity=False)
+    params = st.fixed_dictionaries(dict(
+        tile_length=st.tuples(st.floats(0.5, 4000.0, width=32, **pos), st.floats(0.5, 4000.0, width=32, **pos)),
+        wind_speed=st.floats(0.0001, 60.0, **pos), wind_direction=st.floats(-360.0, 720.0, **pos),
+        fetch_length=st.floats(0.0001, 2000.0, **pos), swell=st.floats(0.0, 2.0, **pos), spread=st.floats(0.0, 1.0, **pos),
+        detail=st.floats(0.0, 1.0, **pos), whitecap=st.floats(0.0, 2.0, **pos), foam_amount=st.floats(0.0, 10.0, **pos),
+        spectrum_seed=st.tuples(st.integers(-2**31, 2**31 - 1), st.integers(-2**31, 2**31 - 1)),
+        time=st.floats(0.0, 50000.0, **pos)))
+    draws = []
+
+    @settings(max_examples=12, deadline=None, derandomize=True, suppress_health_check=[HealthCheck.too_slow])
+    @given(kw=params, contract=st.sampled_from([po.CONTRACT_FMA, po.CONTRACT_STRICT]), delta=st.floats(0.0, 0.1, **pos))
+    def collect(kw, contract, delta):
+        draws.append(dict(params=kw, contract=contract, delta=delta))
+
+    collect()
+    return draws
+
+
+def ref_pins():
+    import test_ref_pins_oracle as t
+    ref = t.REFERENCE
+    out = {"generator": "oracle/_ref: the reference's compute shaders compiled for the CPU"}
+    for N, C, frames in t.BASELINE_CONFIGS:
+        for mode in t.MODES:
+            out[f"baseline/{N}x{C}x{frames}/{mode[0]}"] = t.baseline_config(ref, N, C, frames, mode)
+    for name in sorted(t.EDGE_CASES):
+        for contract in (po.CONTRACT_FMA, po.CONTRACT_STRICT):
+            out[f"corner/{name}/contract{contract}"] = t.parameter_corner(ref, name, contract)
+    out["foam_loop"] = t.foam_loop(ref)[0]
+    out["random"] = []
+    for d in random_draws():
+        d.update(t.random_parameters(ref, t.random_draw_kwargs(d), d["contract"], d["delta"]))
+        out["random"].append(d)
+    return out
+
+
 if __name__ == "__main__":
     os.makedirs(os.path.join(ROOT, "tests", "golden"), exist_ok=True)
     for case in CASES:
@@ -85,3 +132,8 @@ if __name__ == "__main__":
         with open(path, "w") as f:
             json.dump(res, f, indent=1)
         print("wrote", os.path.relpath(path, ROOT), res["frames_crc"][-1], res["query"]["displacement_crc"])
+    path = os.path.join(ROOT, "tests", "golden", "ref_pins", "states.json")
+    os.makedirs(os.path.dirname(path), exist_ok=True)
+    with open(path, "w") as f:
+        json.dump(ref_pins(), f, indent=1)
+    print("wrote", os.path.relpath(path, ROOT))
