@@ -41,6 +41,16 @@ namespace OceanB200
     }
 
     [StructLayout(LayoutKind.Sequential)]
+    public unsafe struct OceanSurfacePoint                          // struct ocean_surface_point (32 B) <- water.gdshader:31-37 inverted
+    {
+        public float height;                                        // surface height above the query point
+        public float source_x, source_z;                            // undisplaced position whose vertex lands over the query point
+        public float residual;                                      // |source + D.xz(source) - q|, metres
+        public fixed float gradient_foam[3];                        // ocean_sample_maps' gradient/foam at the source point
+        public float jacobian;                                      // <= 0: folded surface
+    }
+
+    [StructLayout(LayoutKind.Sequential)]
     public struct OceanInfo
     {
         public int device, map_size, num_cascades, pending_cascades;
@@ -87,6 +97,14 @@ namespace OceanB200
         [LibraryImport(Lib)] [UnmanagedCallConv(CallConvs = new[] { typeof(System.Runtime.CompilerServices.CallConvCdecl) })]
         internal static partial int ocean_sample_maps(IntPtr handle, int num_points, float* points_xz, int num_cascades, float* map_scales,
                                                       float* displacement, float* gradient_foam);
+        // surface query: the map query above world x,z with the horizontal displacement inverted; iterations in [0, 32], 8 = default.
+        // The _device form takes device pointers for points and records and is asynchronous on the generator's stream.
+        [LibraryImport(Lib)] [UnmanagedCallConv(CallConvs = new[] { typeof(System.Runtime.CompilerServices.CallConvCdecl) })]
+        internal static partial int ocean_query_surface(IntPtr handle, int num_points, float* points_xz, int num_cascades, float* map_scales,
+                                                        int iterations, OceanSurfacePoint* points_out);
+        [LibraryImport(Lib)] [UnmanagedCallConv(CallConvs = new[] { typeof(System.Runtime.CompilerServices.CallConvCdecl) })]
+        internal static partial int ocean_query_surface_device(IntPtr handle, int num_points, float* points_xz_dev, int num_cascades,
+                                                               float* map_scales, int iterations, OceanSurfacePoint* points_out_dev);
         // fused frames, overlapped hand-off, Water scheduler, spray candidates (include/ocean.h)
         [LibraryImport(Lib)] [UnmanagedCallConv(CallConvs = new[] { typeof(System.Runtime.CompilerServices.CallConvCdecl) })]
         internal static partial int ocean_update_frames(IntPtr handle, double delta, OceanCascadeParams* parameters, int count, int frames);

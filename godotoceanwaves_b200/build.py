@@ -8,7 +8,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(_HERE, "libocean.so")
-SOURCES = ["ocean_kernels.cu", "ocean_sample.cu", "ocean_spray.cu", "ocean_api.cu"]
+SOURCES = ["ocean_kernels.cu", "ocean_sample.cu", "ocean_spray.cu", "ocean_surface.cu", "ocean_api.cu"]
 HEADERS = ["ocean_kernels.cuh", "ocean_texture.cuh", "detmath.cuh", "fft_core.cuh", os.path.join("..", "..", "include", "ocean.h")]
 
 NVCC_FLAGS = [

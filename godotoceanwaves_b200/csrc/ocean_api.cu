@@ -65,6 +65,8 @@ struct ocean_generator {
     int spray_count_capacity = 0;
     void* spray_records = nullptr;                      // spray op staging for the host entry point
     size_t spray_record_capacity = 0;
+    void* surface_points = nullptr;                     // surface query staging for the host entry point
+    size_t surface_point_capacity = 0;
     ocean::CascadeDispatch* d_cascade = nullptr;        // [num_cascades] (two-kernel path only)
     ocean::SpectrumDispatch* d_spectrum = nullptr;      // [num_cascades]
     ocean::TableDispatch* d_tables = nullptr;           // [num_cascades]
@@ -161,6 +163,7 @@ void release(ocean_generator* g) {
     if (g->snap_free) cudaEventDestroy(g->snap_free);
     cudaFree(g->spray_counts);
     cudaFree(g->spray_records);
+    cudaFree(g->surface_points);
     cudaFree(g->d_cascade);
     cudaFree(g->d_spectrum);
     cudaFree(g->d_queue);
@@ -949,6 +952,18 @@ int upload_scales(ocean_generator* gen, int num_cascades, const float* map_scale
     OCEAN_CUDA(cudaMemcpyAsync(gen->q_scales, map_scales_host, sizeof(float4) * (size_t)num_cascades, cudaMemcpyHostToDevice, gen->stream));
     return OCEAN_OK;
 }
+// Grows the query staging (points and the map query's outputs; the host entry points of every query op share it) to n points.
+int reserve_query_points(ocean_generator* gen, size_t n) {
+    if (n <= gen->q_capacity) return OCEAN_OK;
+    OCEAN_CUDA(cudaStreamSynchronize(gen->stream));
+    cudaFree(gen->q_points); cudaFree(gen->q_disp); cudaFree(gen->q_grad);
+    gen->q_points = nullptr; gen->q_disp = gen->q_grad = nullptr; gen->q_capacity = 0;
+    OCEAN_CUDA(dev_alloc(gen, &gen->q_points, n));
+    OCEAN_CUDA(dev_alloc(gen, &gen->q_disp, 3 * n));
+    OCEAN_CUDA(dev_alloc(gen, &gen->q_grad, 3 * n));
+    gen->q_capacity = n;
+    return OCEAN_OK;
+}
 }  // namespace
 
 int ocean_sample_maps_device(ocean_generator* gen, int num_points, const float* points_xz_dev, int num_cascades, const float* map_scales_host,
@@ -973,15 +988,7 @@ int ocean_sample_maps(ocean_generator* gen, int num_points, const float* points_
     if (num_points == 0) return OCEAN_OK;
     if (!points_xz_host || !displacement_host || !gradient_foam_host) return fail(OCEAN_ERR_INVALID_ARGUMENT, "a host buffer is NULL");
     const size_t n = (size_t)num_points;
-    if (n > gen->q_capacity) {
-        OCEAN_CUDA(cudaStreamSynchronize(gen->stream));
-        cudaFree(gen->q_points); cudaFree(gen->q_disp); cudaFree(gen->q_grad);
-        gen->q_points = nullptr; gen->q_disp = gen->q_grad = nullptr; gen->q_capacity = 0;
-        OCEAN_CUDA(dev_alloc(gen, &gen->q_points, n));
-        OCEAN_CUDA(dev_alloc(gen, &gen->q_disp, 3 * n));
-        OCEAN_CUDA(dev_alloc(gen, &gen->q_grad, 3 * n));
-        gen->q_capacity = n;
-    }
+    if ((rc = reserve_query_points(gen, n))) return rc;
     OCEAN_CUDA(cudaMemcpyAsync(gen->q_points, points_xz_host, sizeof(float2) * n, cudaMemcpyHostToDevice, gen->stream));
     if ((rc = ocean_sample_maps_device(gen, num_points, reinterpret_cast<const float*>(gen->q_points), num_cascades, map_scales_host,
                                        gen->q_disp, gen->q_grad)))
@@ -1062,15 +1069,7 @@ int ocean_extract_spray(ocean_generator* gen, int num_candidates, const float* p
     if (num_candidates == 0) return OCEAN_OK;
     if (!points_xz_host || (max_records > 0 && !records_host)) return fail(OCEAN_ERR_INVALID_ARGUMENT, "a host buffer is NULL");
     const size_t n = (size_t)num_candidates;
-    if (n > gen->q_capacity) {                       // the candidate staging buffer is shared with the map-query op
-        OCEAN_CUDA(cudaStreamSynchronize(gen->stream));
-        cudaFree(gen->q_points); cudaFree(gen->q_disp); cudaFree(gen->q_grad);
-        gen->q_points = nullptr; gen->q_disp = gen->q_grad = nullptr; gen->q_capacity = 0;
-        OCEAN_CUDA(dev_alloc(gen, &gen->q_points, n));
-        OCEAN_CUDA(dev_alloc(gen, &gen->q_disp, 3 * n));
-        OCEAN_CUDA(dev_alloc(gen, &gen->q_grad, 3 * n));
-        gen->q_capacity = n;
-    }
+    if ((rc = reserve_query_points(gen, n))) return rc;    // the candidate staging buffer is shared with the map-query op
     const size_t rec_bytes = ((size_t)max_records + 1) * sizeof(ocean_spray_record);    // + one slot for the count
     if (rec_bytes > gen->spray_record_capacity) {
         OCEAN_CUDA(cudaStreamSynchronize(gen->stream));
@@ -1093,6 +1092,62 @@ int ocean_extract_spray(ocean_generator* gen, int num_candidates, const float* p
     const int kept = count < max_records ? count : max_records;
     if (kept > 0) OCEAN_CUDA(cudaMemcpy(records_host, recs, sizeof(ocean_spray_record) * (size_t)kept, cudaMemcpyDeviceToHost));
     *num_active = count;
+    return OCEAN_OK;
+}
+
+// ---- surface query: the map query above a world position, horizontal displacement inverted ----
+static_assert(sizeof(ocean_surface_point) == 32, "ocean_surface_point layout");
+
+namespace {
+int check_surface_args(int num_points, int iterations) {
+    if (num_points < 0) return fail(OCEAN_ERR_INVALID_ARGUMENT, "num_points %d is negative", num_points);
+    if (iterations < 0 || iterations > OCEAN_SURFACE_MAX_ITERATIONS)
+        return fail(OCEAN_ERR_INVALID_ARGUMENT, "iterations %d outside [0, %d]", iterations, OCEAN_SURFACE_MAX_ITERATIONS);
+    return OCEAN_OK;
+}
+}  // namespace
+
+int ocean_query_surface_device(ocean_generator* gen, int num_points, const float* points_xz_dev, int num_cascades, const float* map_scales_host,
+                               int iterations, ocean_surface_point* out_dev) {
+    OCEAN_ENTER(gen);
+    if (rc) return rc;
+    if ((rc = check_surface_args(num_points, iterations))) return rc;
+    if (num_points == 0) return OCEAN_OK;
+    if (!points_xz_dev || !out_dev) return fail(OCEAN_ERR_INVALID_ARGUMENT, "a device buffer is NULL");
+    if ((rc = upload_scales(gen, num_cascades, map_scales_host))) return rc;
+    OCEAN_CUDA(ocean::launch_query_surface(gen->buf, num_cascades, reinterpret_cast<const float2*>(points_xz_dev), num_points, gen->q_scales,
+                                           iterations, out_dev, gen->stream));
+    gen->kernel_launches += 1;
+    return OCEAN_OK;
+}
+
+int ocean_query_surface(ocean_generator* gen, int num_points, const float* points_xz_host, int num_cascades, const float* map_scales_host,
+                        int iterations, ocean_surface_point* out_host) {
+    OCEAN_ENTER(gen);
+    if (rc) return rc;
+    if ((rc = check_surface_args(num_points, iterations))) return rc;
+    if (num_points == 0) return OCEAN_OK;
+    if (!points_xz_host || !out_host) return fail(OCEAN_ERR_INVALID_ARGUMENT, "a host buffer is NULL");
+    const size_t n = (size_t)num_points;
+    if ((rc = reserve_query_points(gen, n))) return rc;
+    const size_t out_bytes = n * sizeof(ocean_surface_point);
+    if (out_bytes > gen->surface_point_capacity) {
+        OCEAN_CUDA(cudaStreamSynchronize(gen->stream));
+        cudaFree(gen->surface_points);
+        gen->device_bytes -= gen->surface_point_capacity;
+        gen->surface_points = nullptr;
+        gen->surface_point_capacity = 0;
+        OCEAN_CUDA(cudaMalloc(&gen->surface_points, out_bytes));
+        gen->device_bytes += out_bytes;
+        gen->surface_point_capacity = out_bytes;
+    }
+    ocean_surface_point* out_dev = static_cast<ocean_surface_point*>(gen->surface_points);
+    OCEAN_CUDA(cudaMemcpyAsync(gen->q_points, points_xz_host, sizeof(float2) * n, cudaMemcpyHostToDevice, gen->stream));
+    if ((rc = ocean_query_surface_device(gen, num_points, reinterpret_cast<const float*>(gen->q_points), num_cascades, map_scales_host,
+                                         iterations, out_dev)))
+        return rc;
+    OCEAN_CUDA(cudaMemcpyAsync(out_host, out_dev, out_bytes, cudaMemcpyDeviceToHost, gen->stream));
+    OCEAN_CUDA(cudaStreamSynchronize(gen->stream));
     return OCEAN_OK;
 }
 

@@ -118,6 +118,11 @@ cudaError_t launch_rowpass_export(const DeviceBuffers& b, int scratch_layer, flo
 cudaError_t launch_sample_maps(const DeviceBuffers& b, int num_cascades, const float2* points_dev, int n, const float4* scales_dev,
                                float* disp_out_dev, float* grad_out_dev, cudaStream_t stream);
 
+// ocean_surface.cu: surface query (water.gdshader:27-39 inverted, then :72-84 at the solved source point); out_dev receives
+// n ocean_surface_point records
+cudaError_t launch_query_surface(const DeviceBuffers& b, int num_cascades, const float2* points_dev, int n, const float4* scales_dev,
+                                 int iterations, void* out_dev, cudaStream_t stream);
+
 // ocean_spray.cu: spray candidates (sea_spray_particle.gdshader:80-94) as a stable stream compaction; counts_dev is
 // [spray_blocks(n) + 1] ints of scratch whose last element receives the number of active candidates
 int spray_blocks(int n);

@@ -19,33 +19,6 @@ namespace ocean {
 
 namespace {
 
-// water.gdshader:42-51
-__device__ __forceinline__ void cubic_weights(float a, float (&w)[4]) {
-    const float a2 = a * a, a3 = a2 * a;
-    w[0] = (-a3 + a2 * 3.0f - a * 3.0f + 1.0f) / 6.0f;
-    w[1] = (a3 * 3.0f - a2 * 6.0f + 4.0f) / 6.0f;
-    w[2] = (-a3 * 3.0f + a2 * 3.0f + a * 3.0f + 1.0f) / 6.0f;
-    w[3] = a3 / 6.0f;
-}
-
-// water.gdshader:55-70
-__device__ __forceinline__ float4 texture_bicubic(const uint2* __restrict__ layer, int N, float u, float v) {
-    const float dims = (float)N, dims_inv = 1.0f / dims;
-    const float ux = u * dims + 0.5f, vy = v * dims + 0.5f;
-    const float flx = floorf(ux), fly = floorf(vy);
-    float wx[4], wy[4];
-    cubic_weights(ux - flx, wx);
-    cubic_weights(vy - fly, wy);
-    const float gx = wx[0] + wx[1], gy = wx[2] + wx[3], gz = wy[0] + wy[1], gw = wy[2] + wy[3];
-    const float hx = (wx[1] / gx + -1.5f + flx) * dims_inv;
-    const float hy = (wx[3] / gy + 0.5f + flx) * dims_inv;
-    const float hz = (wy[1] / gz + -1.5f + fly) * dims_inv;
-    const float hw = (wy[3] / gw + 0.5f + fly) * dims_inv;
-    const float wxx = gx / (gx + gy), wyy = gz / (gz + gw);
-    return mix4(mix4(texture_bilinear(layer, N, hy, hw), texture_bilinear(layer, N, hx, hw), wxx),
-                mix4(texture_bilinear(layer, N, hy, hz), texture_bilinear(layer, N, hx, hz), wxx), wyy);
-}
-
 __global__ void __launch_bounds__(256) k_sample_maps(const uint2* __restrict__ displacement, const uint2* __restrict__ normal, int N, int C,
                                                      const float2* __restrict__ points, int n, const float4* __restrict__ scales,
                                                      float* __restrict__ disp_out, float* __restrict__ grad_out) {
@@ -61,9 +34,7 @@ __global__ void __launch_bounds__(256) k_sample_maps(const uint2* __restrict__ d
         dx = dx + d.x * s.z;
         dy = dy + d.y * s.z;
         dz = dz + d.z * s.z;
-        const float ppm = (float)N * fminf(s.x, s.y);                                             // :80
-        const float t = fminf(1.0f, ppm * 0.1f);
-        const float4 m = mix4(texture_bicubic(normal + layer, N, u, v), texture_bilinear(normal + layer, N, u, v), t);   // :83
+        const float4 m = normal_sample(normal + layer, N, s, u, v);                               // :80-83
         gx = gx + m.x * s.w;
         gy = gy + m.y * s.w;
         gf = gf + m.w * 1.0f;

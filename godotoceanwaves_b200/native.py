@@ -71,6 +71,8 @@ SIGNATURES = {
     "ocean_debug_work_queue": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int]),
     "ocean_sample_maps": (C.c_int, [_H, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ocean_sample_maps_device": (C.c_int, [_H, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "ocean_query_surface": (C.c_int, [_H, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
+    "ocean_query_surface_device": (C.c_int, [_H, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "ocean_spray_grid": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p]),
     "ocean_extract_spray": (C.c_int, [_H, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, _P(C.c_int)]),
     "ocean_extract_spray_device": (C.c_int, [_H, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),

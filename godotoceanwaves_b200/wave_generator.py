@@ -230,6 +230,23 @@ class WaveGenerator:
                                                disp.ctypes.data, grad.ctypes.data))
         return disp, grad
 
+    # -- surface query: the map query above a world position, the horizontal displacement of water.gdshader:31-37 inverted --
+    SURFACE_POINT = np.dtype([("height", np.float32), ("source_x", np.float32), ("source_z", np.float32), ("residual", np.float32),
+                              ("gradient_foam", np.float32, 3), ("jacobian", np.float32)])      # struct ocean_surface_point
+
+    def query_surface(self, points_xz, map_scales, iterations: int = 8) -> np.ndarray:
+        """The water surface above the world positions points_xz [n][2] as SURFACE_POINT rows: height, the undisplaced
+        source point whose displaced vertex lands there, the residual |source + D.xz(source) - q| in metres, the
+        gradient/foam of sample() at the source point and the Jacobian determinant there (<= 0: folded surface).
+        `iterations` damped Newton steps (0..32) solve source + D.xz(source) = q; see ocean_query_surface in ocean.h."""
+        self._require()
+        pts = np.ascontiguousarray(points_xz, np.float32).reshape(-1, 2)
+        sc = np.ascontiguousarray(map_scales, np.float32).reshape(-1, 4)
+        out = np.empty(pts.shape[0], self.SURFACE_POINT)
+        check(load_library().ocean_query_surface(self.context, pts.shape[0], pts.ctypes.data, sc.shape[0], sc.ctypes.data, int(iterations),
+                                                 out.ctypes.data))
+        return out
+
     # -- spray candidates: the spawn test of sea_spray_particle.gdshader:80-94 as a stream compaction --------------
     SPRAY_RECORD = np.dtype([("index", np.uint32), ("start_x", np.float32), ("start_z", np.float32), ("scale_factor", np.float32),
                              ("particle_scale", np.float32, 3), ("foam", np.float32)])     # struct ocean_spray_record
